@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      (the CPU oracle port of the reference path, host cores)
+    python bench.py ... --dump-outputs DIR    (also writes the last timed step's keypoints + argmax as DIR/*.npy)
 
 A step = one pass of the hot path over one batch of synthetic crops per GPU:
     crops f32 [B,3,256,192] (resident in HBM) -> ViT-B -> head -> heatmaps -> decode -> keypoints [B,K,3]
@@ -403,6 +404,16 @@ def stream_workload(rank: int, frames: int, max_n: int):
     return imgs, boxes, counts
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy in float32 / float64.  The inputs and weights are seeded, so two builds run
+    with the same arguments can be compared output for output."""
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "outputs to dump exceed 64 MB"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu(args) -> None:
     import torch
     import torch.distributed as dist
@@ -448,7 +459,7 @@ def run_gpu(args) -> None:
                    "weights + activations touched per step exceed L2 several times over")
 
         def step(i: int):
-            kp, _ = model.infer_crops(crops[i % NBUF], org_wh)
+            kp, idx = model.infer_crops(crops[i % NBUF], org_wh)
             if world > 1:
                 # the path's only exchange: final keypoints, gathered on a side stream so it never sits between two
                 # steps of the compute stream (13 KB per rank: pure latency)
@@ -457,7 +468,7 @@ def run_gpu(args) -> None:
                 with torch.cuda.stream(comm):
                     kp.record_stream(comm)
                     dist.all_gather_into_tensor(gathered, kp)
-            return kp
+            return [(kp, idx)]
     else:
         # configs[4]: one video stream per GPU; a step = `streams` consecutive frames, each with its own ragged crop batch,
         # through the frame-level entry point (uint8 frame + boxes resident in HBM -> frame keypoints)
@@ -474,10 +485,7 @@ def run_gpu(args) -> None:
                    f"({int(counts.min())}..{int(counts.max())} crops, {crops_per_step} per step on rank 0's stream)")
 
         def step(i: int):
-            kp = None
-            for f in range(streams):
-                kp, _ = model.infer_frame(d_imgs[(i * streams + f) % 4], d_boxes[f])
-            return kp
+            return [model.infer_frame(d_imgs[(i * streams + f) % 4], d_boxes[f]) for f in range(streams)]
 
     def barrier():
         if world > 1:
@@ -508,12 +516,19 @@ def run_gpu(args) -> None:
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         step(i)
+    last = step(args.steps - 1)
     if comm is not None:
         torch.cuda.current_stream().wait_stream(comm)          # the last gathers are part of the timed work
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # (keypoints, argmax) of every call in the last timed step, as the caller received them
+        outputs = {"keypoints": torch.cat([kp for kp, _ in last]), "argmax": torch.cat([idx for _, idx in last]).double()}
+        if world > 1 and not streams:
+            outputs["keypoints_all_ranks"] = gathered
+        dump_outputs(args.dump_outputs, {name: t.cpu().numpy() for name, t in outputs.items()})
     ms_total = ev0.elapsed_time(ev1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -745,11 +760,17 @@ def main() -> None:
     ap.add_argument("--no-frame-path", action="store_true", help="skip the frame-level (f1/f2) section of the N=1 line")
     ap.add_argument("--config", default=None, choices=list(CONFIGS), help="BASELINE.json configs[1..4] presets (override --model/--keypoints/--batch)")
     ap.add_argument("--stream-frames", type=int, default=0, help="video-stream mode: frames (ragged crop batches) per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the keypoints and argmax the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
     if args.config:
         c = CONFIGS[args.config]
         args.model, args.keypoints, args.batch = c["model"], c["keypoints"], c["batch"]
         args.stream_frames = c.get("streams", 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

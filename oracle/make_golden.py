@@ -1,6 +1,7 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference  --  TEST INFRASTRUCTURE ONLY.
 
 Run here (the container that has /root/reference):   python oracle/make_golden.py
+Only some cases:   python oracle/make_golden.py h_wholebody decode_crop
 The reference is a Python package and cannot travel to the GPU box, so its outputs on seeded
 inputs are committed as small fixtures.  Inputs and weights are NOT stored: both sides
 regenerate them from the seeds with oracle.vitpose_oracle.make_state_dict / make_crops /
@@ -8,7 +9,8 @@ make_decode_maps (np.random.RandomState is a frozen stream).
 
 What is pinned:
   fwd_<size>_<dataset>.npz  reference ViTPose(cfg).forward heatmaps (vit_models/model.py:23-24)
-                            + VitInference.postprocess keypoints (easy_ViTPose/inference.py:187-205)
+                            + VitInference.postprocess keypoints (easy_ViTPose/inference.py:187-205);
+                            heatmaps too large for one file below 1 MB continue in fwd_<...>.part<i>.npz (oracle/golden_io.py)
   decode_crop.npz           keypoints_from_heatmaps called per crop (N=1), as VitInference does
   decode_batch.npz          keypoints_from_heatmaps called once on an [N,K,H,W] batch
   blur_check                asserted here: oracle blur == cv2.GaussianBlur bit for bit
@@ -23,7 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle import ref_import, vitpose_oracle as O  # noqa: E402
+from oracle import golden_io, ref_import, vitpose_oracle as O  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 
@@ -37,7 +39,7 @@ FORWARD_CASES = {
 DECODE_CASES = {"decode_crop": (6, 17, 301), "decode_batch": (3, 25, 302)}
 
 
-def main() -> None:
+def main(only: list[str]) -> None:
     import cv2
     import torch
     torch.set_grad_enabled(False)
@@ -56,6 +58,8 @@ def main() -> None:
     print("blur order: bit-exact vs cv2", cv2.__version__)
 
     for name, (size, dataset, K, B, wseed, xseed, org, peaky) in FORWARD_CASES.items():
+        if only and name not in only:
+            continue
         D, depth, heads = O.MODEL_DIMS[size]
         cfg = ns.dyn_model_import(dataset, size)
         model = ns.ViTPose(cfg).eval()
@@ -66,12 +70,14 @@ def main() -> None:
         org_wh = np.array(org, np.int32)
         kp = np.concatenate([ref_import.postprocess(ns, hm[i:i + 1], int(org_wh[i, 0]), int(org_wh[i, 1]))
                              for i in range(B)], 0).astype(np.float32)
-        np.savez_compressed(os.path.join(OUT, f"fwd_{name}.npz"), heatmaps=hm, kpts=kp, org_wh=org_wh,
-                            meta=np.array([D, depth, heads, K, B, wseed, xseed], np.int64), peaky=np.float64(peaky))
+        golden_io.save(os.path.join(OUT, f"fwd_{name}.npz"), dict(heatmaps=hm, kpts=kp, org_wh=org_wh,
+                       meta=np.array([D, depth, heads, K, B, wseed, xseed], np.int64), peaky=np.float64(peaky)), split_key="heatmaps")
         print(name, "heatmap range", float(hm.min()), float(hm.max()),
               "positive maxima", int((hm.reshape(B, K, -1).max(-1) > 0).sum()), "/", B * K)
 
     for name, (N, K, seed) in DECODE_CASES.items():
+        if only and name not in only:
+            continue
         maps = O.make_decode_maps(N, K, seed)
         rs = np.random.RandomState(seed + 1)
         org_wh = np.stack([rs.randint(64, 513, size=N), rs.randint(64, 513, size=N)], 1).astype(np.int32)
@@ -93,4 +99,4 @@ def main() -> None:
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

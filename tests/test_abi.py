@@ -3,6 +3,9 @@ mirror of the reference interface behaves (no GPU compute here)."""
 import ctypes
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -25,15 +28,23 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from easy_vitpose_b200 import ViTPose, decode_heatmaps, model_cfg
-    m = ViTPose(model_cfg("b", 17))
-    with pytest.raises(RuntimeError):
-        m.to("cpu")
-    with pytest.raises(RuntimeError):
-        decode_heatmaps(torch.zeros(1, 17, 64, 48), torch.tensor([[192, 256]]))
+    """Runs in a child process with every GPU hidden (CUDA_VISIBLE_DEVICES=""), so a machine with a GPU checks it too."""
+    code = textwrap.dedent("""
+        import torch
+        assert not torch.cuda.is_available()
+        from easy_vitpose_b200 import ViTPose, decode_heatmaps, model_cfg
+        m = ViTPose(model_cfg("b", 17))
+        for call in (lambda: m.to("cpu"), lambda: decode_heatmaps(torch.zeros(1, 17, 64, 48), torch.tensor([[192, 256]]))):
+            try:
+                call()
+            except RuntimeError:
+                continue
+            raise AssertionError("no RuntimeError without a GPU")
+        print("raised")
+    """)
+    out = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0 and out.stdout.split() == ["raised"], out.stdout + out.stderr[-2000:]
 
 
 def test_configs_match_reference_shapes():

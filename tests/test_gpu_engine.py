@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import vitpose_oracle as O
+from oracle import golden_io, vitpose_oracle as O
 
 pytestmark = pytest.mark.gpu
 
@@ -29,7 +29,7 @@ def _engine(g, max_batch=8):
 
 @pytest.mark.parametrize("name", ["s_coco", "b_coco", "l_coco_25", "h_wholebody"])
 def test_forward_heatmaps_vs_reference(golden_dir, name):
-    g = np.load(os.path.join(golden_dir, f"fwd_{name}.npz"))
+    g = golden_io.load(os.path.join(golden_dir, f"fwd_{name}.npz"))
     m, x = _engine(g)
     hm = m(torch.from_numpy(x).cuda()).cpu().numpy()
     ref = g["heatmaps"]

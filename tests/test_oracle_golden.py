@@ -5,13 +5,13 @@ import os
 import numpy as np
 import pytest
 
-from oracle import ref_import, vitpose_oracle as O
+from oracle import golden_io, vitpose_oracle as O
 
 FWD = ["s_coco", "b_coco", "l_coco_25", "h_wholebody"]
 
 
 def _load(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name + ".npz"))
+    return golden_io.load(os.path.join(golden_dir, name + ".npz"))
 
 
 @pytest.mark.parametrize("name", FWD)
@@ -53,13 +53,14 @@ def test_decode_edge_cases(golden_dir, name, wrap):
     assert np.all(err[~well] <= 1e-3 + 1e-3 * np.abs(ref[~well]))
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree only exists in the build container")
-def test_live_reference_decode_matches_oracle():
-    ns = ref_import.load()
-    maps = O.make_decode_maps(2, 17, 999)
-    for i in range(2):
-        ref = ref_import.postprocess(ns, maps[i:i + 1], 200 + i, 300 + i)
-        kp, _ = O.decode_maps(maps[i:i + 1], np.array([[200 + i, 300 + i]]), wrap="crop")
+def test_reference_postprocess_matches_oracle(golden_dir):
+    """VitInference.postprocess of the unmodified reference, one crop per call (oracle/make_golden_ref_calls.py)."""
+    g = _load(golden_dir, "decode_postprocess")
+    N, K, seed = (int(v) for v in g["meta"])
+    maps = O.make_decode_maps(N, K, seed)
+    for i in range(N):
+        ref = g["kpts"][i]
+        kp, _ = O.decode_maps(maps[i:i + 1], g["org_wh"][i:i + 1], wrap="crop")
         assert np.array_equal(kp[..., 2], ref[..., 2])
         assert np.abs(kp - ref).max() < 1e-3 + 1e-3 * np.abs(ref).max()
 

@@ -1,11 +1,16 @@
 """CPU: oracle/preproc_oracle.py (SURVEY.md section 8 row f1) against the fixtures the UNMODIFIED reference produced
-(oracle/make_golden_frames.py), against cv2 where it is installed, and against the reference tree where it is mounted."""
+(oracle/make_golden_frames.py, oracle/make_golden_ref_calls.py), including what cv2.resize returns."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
-from oracle import preproc_oracle as P, ref_import
+from oracle import preproc_oracle as P
+
+
+def _sha256(a):
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
 
 
 def _case(golden_dir, name):
@@ -49,13 +54,16 @@ def test_padded_box_clips_to_frame():
     assert P.padded_box((300, 300, 310, 310), 100, 200) == (200, 100, 200, 100)      # empty: the reference raises later
 
 
-def test_resize_matches_cv2_on_random_sizes():
-    cv2 = pytest.importorskip("cv2")
+def test_resize_matches_cv2_on_random_sizes(golden_dir):
+    """cv2.resize(img, (192, 256), INTER_LINEAR) outputs, pinned by their SHA-256 digests (tests/golden/resize_cv2.npz)."""
+    g = np.load(os.path.join(golden_dir, "resize_cv2.npz"))
     rs = np.random.RandomState(0)
     sizes = [(rs.randint(1, 700), rs.randint(1, 600)) for _ in range(25)] + [(256, 192), (512, 384), (1, 1), (2, 3), (1080, 810)]
-    for h, w in sizes:
+    assert np.array_equal(np.array(sizes), g["sizes"])
+    for (h, w), want in zip(sizes, g["sha256"]):
         img = rs.randint(0, 256, size=(h, w, 3), dtype=np.uint8)
-        assert np.array_equal(P.resize_linear_u8(img), cv2.resize(img, (192, 256), interpolation=cv2.INTER_LINEAR)), (h, w)
+        r = P.resize_linear_u8(img)
+        assert r.dtype == np.uint8 and r.shape == (256, 192, 3) and np.array_equal(_sha256(r), want), (h, w)
 
 
 def test_to_frame_coords_is_one_rounding():
@@ -67,21 +75,19 @@ def test_to_frame_coords_is_one_rounding():
     assert np.array_equal(out[..., 2], kp[..., 2])
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted (GPU box)")
-def test_against_reference_pad_image_and_pre_img():
-    cv2 = pytest.importorskip("cv2")
-    inf = ref_import.load_vitinference()
-    rs = np.random.RandomState(2)
-    frame = P.make_frame(200, 260, 5)
-    stub = type("S", (), {"target_size": (192, 256)})()
-    for _ in range(12):
-        x0, y0 = rs.randint(-20, 240), rs.randint(-20, 180)
-        box = np.array([x0, y0, x0 + rs.randint(1, 150), y0 + rs.randint(1, 150)])
-        bx0, by0, bx1, by1 = P.padded_box(box, 200, 260)
-        if bx1 <= bx0 or by1 <= by0:
-            continue
-        padded, (left, top) = inf.pad_image(frame[by0:by1, bx0:bx1], 3 / 4)
+def test_against_reference_pad_image_and_pre_img(golden_dir):
+    """The reference's pad_image and VitInference.pre_img on seeded boxes (oracle/make_golden_ref_calls.py): canvas and
+    network input are pinned bit for bit through their SHA-256 digests."""
+    g = np.load(os.path.join(golden_dir, "pad_pre_img.npz"))
+    fh, fw, fseed = (int(v) for v in g["meta"][:3])
+    frame = P.make_frame(fh, fw, fseed)
+    assert len(g["boxes"]) == 12
+    for n, box in enumerate(g["boxes"]):
+        bx0, by0, _, _ = P.padded_box(box, fh, fw)
+        left, top = (int(v) for v in g["left_top"][n])
         canvas, off = P.crop_canvas(frame, box)
-        assert np.array_equal(canvas, padded) and off == (by0 - top, bx0 - left)
-        x, org_h, org_w = inf.VitInference.pre_img(stub, padded)
-        assert np.array_equal(P.pre_img(canvas), x) and (org_h, org_w) == canvas.shape[:2]
+        assert canvas.shape == tuple(g["canvas_shape"][n]) and np.array_equal(_sha256(canvas), g["canvas_sha256"][n])
+        assert off == (by0 - top, bx0 - left)
+        x = P.pre_img(canvas)
+        assert x.dtype == np.float32 and x.shape == tuple(g["x_shape"][n]) and np.array_equal(_sha256(x), g["x_sha256"][n])
+        assert tuple(g["org_hw"][n]) == canvas.shape[:2]
